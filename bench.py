@@ -2,6 +2,7 @@
 """bench.py -- LLaMA-7B Q4_0 tokens/sec on B200 (BASELINE.json metric): decode@1 (default line) and prefill@512 (--metric prefill).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--metric decode|prefill]    our arm (N>1: torchrun, one replica per GPU)
+  python bench.py ... --dump-outputs DIR                                          also write the logits of the last timed step as DIR/*.npy
   python bench.py --impl reference [--metric decode|prefill] [...]                  the reference's own ggml CPU path, FULL 32-layer model
 
 A "step" is one pass of the hot path over one batch: one decode token (Llama::evaluate with 1 token) at n_past = 512 on a
@@ -261,6 +262,14 @@ MODELS = {"7b-q4_0": dict(HP_7B), "13b-q5_1": dict(n_vocab=32000, n_embd=5120, n
 BLK_BYTES = {2: 18, 3: 20, 6: 22, 7: 24, 8: 34}
 
 
+def dump_outputs(d, **arrays):
+    """--dump-outputs: the arrays a caller of the timed path received in its last step, as float32 .npy files.  The model and the prompt are
+    seeded, so two builds run with the same arguments can be compared output for output."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, np.float32))
+
+
 def tp_main(args, rank, local_rank, world, steps, warmup, emit, log):
     """decode@1 at n_past = 512 of ONE model sharded by output rows over the N GPUs (strong scaling): every rank streams 1/N of the weights and its
     heads' KV cache; activation slices cross NVLink as peer stores issued by the producing kernels' epilogues as tagged 8-byte units {payload, tag} the consumers poll locally
@@ -371,6 +380,8 @@ def tp_main(args, rank, local_rank, world, steps, warmup, emit, log):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, decode_logits=logits)
     pk = peaks()
     blk = BLK_BYTES[hp["wtype"]]
     wbytes, kvbytes, embbytes = algorithmic_bytes_per_token(hp, N_PAST, blk)
@@ -420,7 +431,11 @@ def main():
     ap.add_argument("--layers", type=int, default=32, help="debug only: anything but 32 is NOT the benchmark config")
     ap.add_argument("--parallel", default="tp", choices=["tp", "replicas"], help="N > 1: tensor-parallel row split of ONE model (strong scaling, default) or N independent replicas")
     ap.add_argument("--model", default="7b-q4_0", choices=["7b-q4_0", "13b-q5_1"], help="13b-q5_1 = BASELINE.json configs[3] (tensor-parallel decode only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="our arm: after the timed steps, write the logits of the last timed step (prefill: the last "
+                    "row of the 512-token evaluate; decode: the token at n_past=512) as DIR/prefill_last_row_logits.npy, DIR/decode_logits.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE line (the JSON); libraries that print to fd 1 (e.g. NCCL's version banner) are sent to stderr
     sys.stdout.flush()
     json_fd = os.dup(1)
@@ -432,7 +447,7 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     prefill_metric = args.metric == "prefill"
-    steps = args.steps if args.steps else (10 if prefill_metric else 64)
+    steps = args.steps if args.steps is not None else (10 if prefill_metric else 64)
     warmup = max(3, args.warmup if args.warmup is not None else (3 if prefill_metric else 8))
     metric_name = METRIC_PREFILL if prefill_metric else METRIC
     workload = ("LLaMA-7B Q4_0 prefill batch=512 from an empty session (BASELINE.json configs[2])" if prefill_metric
@@ -610,6 +625,8 @@ def main():
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, prefill_last_row_logits=last_row, decode_logits=logits)
 
     wbytes, kvbytes, embbytes = algorithmic_bytes_per_token(hp, N_PAST)
     tok_bytes = wbytes + kvbytes + embbytes

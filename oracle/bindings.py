@@ -421,6 +421,13 @@ class OracleLlama:
             return logits, tap
         return logits
 
+    def eval_into(self, tokens, logits):
+        """same as eval, into a caller-owned [n, n_vocab] f32 buffer (RefLlama's interface, used by bench.py's CPU arm)"""
+        tokens = np.ascontiguousarray(tokens, np.int32)
+        rc = self.orc.lib.or_llama_eval(self.m, _p(tokens), tokens.size, _p(logits))
+        assert rc == 0, rc
+        return logits
+
     def eval_tap(self, tokens, il, stage, count):
         """eval and return (logits, flat f32 tap of `count` floats taken at (layer il, stage)); see llama_oracle.c"""
         tokens = np.ascontiguousarray(tokens, np.int32)
@@ -431,6 +438,12 @@ class OracleLlama:
         self.orc.lib.or_llama_set_tap_stage(self.m, None, -2, 11)
         assert rc == 0
         return logits, tap
+
+    def kv_ptr(self, which):
+        """(address, nbytes) of the f16 K (0) / V (1) cache, as RefLlama.kv_ptr"""
+        nb = C.c_size_t(0)
+        p = self.orc.lib.or_llama_kv(self.m, which, C.byref(nb))
+        return p, nb.value
 
     def kv(self, which):
         nb = C.c_size_t(0)

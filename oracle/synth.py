@@ -85,6 +85,23 @@ def make_llama_random_blocks(hp, wtype, seed=0x5EED0000):
     return hp, out
 
 
+# byte offsets of the fp16 super-block scale d (and dmin) in block_q2_K .. block_q6_K (LC/k_quants.h)
+KQUANT_FP16_FIELDS = {B.Q2_K: (80, 82), B.Q3_K: (108,), B.Q4_K: (0, 2), B.Q5_K: (0, 2), B.Q6_K: (208,)}
+
+
+def make_kquant_blocks(t, n, k, seed):
+    """[n, k/256 * block bytes] uint8 rows of K-quant type t drawn directly: uniform bytes for the quants and the packed sub-block scales and
+    mins (every bit pattern is a valid block), fp16 d / dmin ~ U[0.5, 1.5] / 1024.  Weights for the K-quant kernel tests without the
+    reference's quantizer; the expected products of these rows are recorded from the reference (oracle/gen_reference_outputs.py)."""
+    rng = np.random.default_rng(seed)
+    bb, nb = B.SUPER_BLOCK_BYTES[t], k // 256
+    blk = rng.integers(0, 256, size=(n, nb, bb), dtype=np.uint8)
+    for off in KQUANT_FP16_FIELDS[t]:
+        d = ((rng.random((n, nb), dtype=np.float32) + 0.5) / np.float32(1024.0)).astype(np.float16)
+        blk[:, :, off:off + 2] = d.view(np.uint8).reshape(n, nb, 2)
+    return blk.reshape(n, nb * bb)
+
+
 def make_tokens(hp, n, seed=0x70CE11):
     return np.random.default_rng(seed).integers(0, hp["n_vocab"], size=n, dtype=np.int32)
 

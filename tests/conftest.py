@@ -1,3 +1,5 @@
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -37,14 +39,29 @@ def orc():
 
 @pytest.fixture(scope="session")
 def ref():
-    """The reference's own compiled ggml.c (oracle/_ref). Built here when /root/reference exists; prebuilt on the GPU box."""
+    """The reference's own compiled ggml.c (oracle/_ref), which build() makes only where the reference's sources are at hand."""
     from oracle import bindings as B
     if not B.have_ref("ref"):
-        if os.path.exists("/root/reference/crates/ggml/sys/llama-cpp/ggml.c"):
-            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"])
-        else:
-            pytest.skip("oracle/_ref/libggml_ref.so not present and /root/reference absent")
+        pytest.skip("oracle/_ref/libggml_ref.so not built (needs the reference's sources)")
     return B.RefLib("ref")
+
+
+def fingerprint(a):
+    """How tests/golden/reference_outputs.json records an output of the reference: dtype, size and the SHA-256 of the bytes."""
+    a = np.ascontiguousarray(a)
+    return {"dtype": str(a.dtype), "size": int(a.size), "sha256": hashlib.sha256(a.tobytes()).hexdigest()}
+
+
+@pytest.fixture(scope="session")
+def reference():
+    """reference(key, got) asserts that `got` is, bit for bit, what the reference's compiled ggml.c returned for the same seeded inputs
+    (recorded by oracle/gen_reference_outputs.py)."""
+    table = json.load(open(os.path.join(GOLDEN, "reference_outputs.json")))
+
+    def check(key, got):
+        want, mine = table[key], fingerprint(got)
+        assert mine == want, f"{key}: not bit-identical to the reference ({mine['dtype']}[{mine['size']}] vs {want['dtype']}[{want['size']}])"
+    return check
 
 
 @pytest.fixture(scope="session")

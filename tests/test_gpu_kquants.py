@@ -1,9 +1,12 @@
-"""K-quant weights (Q2_K .. Q6_K, SURVEY.md 8f-4) through the C ABI, BIT-EXACT against the reference's own compiled k_quants.c (oracle/_ref):
-quantize_row_q8_K, ggml_vec_dot_q{2..6}_K_q8_K behind ggml_compute_forward_mul_mat, and the same node through the ggml_cuda_* seam."""
+"""K-quant weights (Q2_K .. Q6_K, SURVEY.md 8f-4) through the C ABI, BIT-EXACT against the reference's own compiled k_quants.c:
+quantize_row_q8_K, ggml_vec_dot_q{2..6}_K_q8_K behind ggml_compute_forward_mul_mat, and the same node through the ggml_cuda_* seam.
+The weights are seeded random super-blocks (oracle/synth.make_kquant_blocks); what the reference returned for them is recorded in
+tests/golden/reference_outputs.json."""
 import numpy as np
 import pytest
 
 from oracle import bindings as B
+from oracle import synth
 
 pytestmark = pytest.mark.gpu
 
@@ -31,11 +34,6 @@ def ctx():
     c.close()
 
 
-def kquantize(ref, t, w):
-    """quantize_row_q*_K (the type's from_float) of every row -> uint8 [N, K/256 * block bytes]"""
-    return np.stack([ref.from_float(t, row) for row in np.ascontiguousarray(w, np.float32)])
-
-
 def acts(rng, Bn, K):
     x = (rng.standard_normal((Bn, K)) * rng.uniform(0.05, 8, (Bn, 1))).astype(np.float32)
     if Bn > 2:
@@ -45,47 +43,55 @@ def acts(rng, Bn, K):
     return x
 
 
-def test_quantize_q8_K_bit_exact(L, ref):
-    rng = np.random.default_rng(11)
-    K, Bn = 4096, 9
-    x = acts(rng, Bn, K)
-    got = np.empty((Bn, K // 256 * 292), np.uint8)
+def q8_K_inputs():
+    return acts(np.random.default_rng(11), 9, 4096)
+
+
+def test_quantize_q8_K_bit_exact(L, reference):
+    x = q8_K_inputs()
+    Bn, K = x.shape
+    got = np.empty((Bn, K // 256, 292), np.uint8)
     assert L.b200_op_quantize_q8_K(x.ctypes.data, K, Bn, got.ctypes.data) == 0
-    for b in range(Bn):
-        want = ref.from_float(B.Q8_K, x[b]).reshape(-1, 292)
-        g = got[b].reshape(-1, 292)
-        zero = want[:, :4].copy().view(np.float32)[:, 0] == 0.0            # the reference leaves bsums of an all-zero super-block unwritten
-        assert np.array_equal(g[:, :260], want[:, :260]), b
-        assert np.array_equal(g[~zero, 260:], want[~zero, 260:]), b
+    zero = got[:, :, :4].copy().view(np.float32)[:, :, 0] == 0.0             # the reference leaves bsums of an all-zero super-block unwritten:
+    got[zero, 260:] = 0                                                     # they are recorded as zeros
+    reference("kquant/quantize_q8_K", got)
+
+
+MUL_MAT_SHAPES = [(4096, 130, 1), (11008 // 256 * 256, 64, 1), (256, 33, 5), (5120, 96, 7), (1024, 257, 33)]
+
+
+def mul_mat_inputs(t, K, N, Bn):
+    seed = K * 3 + N + t
+    return synth.make_kquant_blocks(t, N, K, seed), acts(np.random.default_rng(seed), Bn, K)
 
 
 @pytest.mark.parametrize("name,t", KTYPES)
-@pytest.mark.parametrize("K,N,Bn", [(4096, 130, 1), (11008 // 256 * 256, 64, 1), (256, 33, 5), (5120, 96, 7), (1024, 257, 33)])
-def test_mul_mat_kquant_bit_exact(L, ref, name, t, K, N, Bn):
-    rng = np.random.default_rng(K * 3 + N + t)
-    w = (rng.standard_normal((N, K)) / np.sqrt(K)).astype(np.float32)
-    w[:, :16] *= 8.0                                       # spread of sub-block scales / mins
-    x = acts(rng, Bn, K)
-    wq = kquantize(ref, t, w)
-    want = ref.mul_mat(t, wq, x)
+@pytest.mark.parametrize("K,N,Bn", MUL_MAT_SHAPES)
+def test_mul_mat_kquant_bit_exact(L, reference, name, t, K, N, Bn):
+    wq, x = mul_mat_inputs(t, K, N, Bn)
     got = np.empty((Bn, N), np.float32)
     assert L.b200_op_mul_mat(t, wq.ctypes.data, K, N, x.ctypes.data, Bn, got.ctypes.data, 0) == 0
-    assert np.array_equal(got.view(np.uint32), want.view(np.uint32)), (name, K, N, Bn, float(np.abs(got - want).max()))
+    reference(f"kquant/mul_mat/{name}/K{K} N{N} B{Bn}", got)
+
+
+def seam_inputs(t):
+    """-> weights [96, 1024] and the activations of batches 1, 4 and 33"""
+    rng = np.random.default_rng(17 + t)
+    K, N = 1024, 96
+    return synth.make_kquant_blocks(t, N, K, 17 + t), [rng.standard_normal((Bn, K)).astype(np.float32) for Bn in (1, 4, 33)]
 
 
 @pytest.mark.parametrize("name,t", KTYPES)
-def test_seam_mul_mat_kquant(ctx, ref, name, t):
+def test_seam_mul_mat_kquant(ctx, reference, name, t):
     """the node the reference executor sends: src0 uploaded with ggml_cuda_transform_tensor (GGML super-blocks as they are), src1 / dst on the host"""
-    rng = np.random.default_rng(17 + t)
-    K, N = 1024, 96
-    wq = kquantize(ref, t, (rng.standard_normal((N, K)) / np.sqrt(K)).astype(np.float32))
-    for Bn in (1, 4, 33):
-        x = rng.standard_normal((Bn, K)).astype(np.float32)
+    wq, xs = seam_inputs(t)
+    N, K = wq.shape[0], xs[0].shape[1]
+    for x in xs:
         w = ctx.transfer_to_gpu(ctx.quantized(t, wq, K))
         dst = ctx.op_mul_mat(w, ctx.from_numpy(x))
         assert ctx.compute(dst, nth=4) is True
-        got = ctx.host_array(dst).reshape(Bn, N)
-        assert np.array_equal(got.view(np.uint32), ref.mul_mat(t, wq, x).view(np.uint32))
+        got = ctx.host_array(dst).reshape(x.shape[0], N)
+        reference(f"kquant/seam/{name}/B{x.shape[0]}", got)
 
 
 def test_kquant_rejects_bad_shapes(L):

@@ -1,11 +1,15 @@
 """The lane arithmetic of llm_b200/csrc/kquants.cu restated word for word in Python (uint32 shifts / masks, dp4a with signed bytes, the xor-shuffle
 reductions, lane = 8 * part + L) and checked against oracle/kquants_np.py, which tests/test_oracle_kquants.py pins to the reference's compiled k_quants.c.
 CPU only: it guards the index / mask expressions of the CUDA kernel (all five K-quant types) independently of a GPU run."""
+import os
+
 import numpy as np
 import pytest
 
 from oracle import bindings as B
 from oracle import kquants_np as KN
+
+from conftest import GOLDEN
 
 f32 = np.float32
 M = 0xffffffff
@@ -85,15 +89,20 @@ def kernel_row(t,wrow,xblocks):
     return v[0]
 
 
-@pytest.mark.parametrize("name,t", list(B.KQUANT_TYPES.items()))
-def test_kernel_lane_arithmetic_matches_the_pinned_restatement(ref, name, t):
+def lane_inputs():
     rng = np.random.default_rng(5)
     K = 512
     x = (rng.standard_normal((2, K)) * rng.uniform(0.1, 5, (2, 1))).astype(f32)
     x[1] = np.round(x[1] * 4) / 4
     w = (rng.standard_normal((3, K)) / 22).astype(f32)
     w[:, :16] *= 8
-    wq = np.stack([ref.from_float(t, r) for r in w])
+    return x, w
+
+
+@pytest.mark.parametrize("name,t", list(B.KQUANT_TYPES.items()))
+def test_kernel_lane_arithmetic_matches_the_pinned_restatement(name, t):
+    x, _ = lane_inputs()
+    wq = np.load(os.path.join(GOLDEN, "kquants_ref.npz"))[f"lane_{name}_wq"]      # the reference's quantize_row_{name} of lane_inputs()'s w
     for b in range(2):
         xq = KN.quantize_row_q8_K(x[b])
         for n in range(3):

@@ -1,5 +1,5 @@
-"""Pins the oracle: (1) the plain-C restatement against the golden vectors generated from the reference's own
-compiled ggml.c (oracle/gen_golden.py) and (2), when oracle/_ref is present, against that reference run live.
+"""Pins the oracle: the plain-C restatement against what the reference's own compiled ggml.c returned for the same seeded inputs --
+(1) the golden vectors of oracle/gen_golden.py and (2) the recorded outputs of oracle/gen_reference_outputs.py.
 Bit-exact everywhere (integer/byte work and f32 with the reference's own operation order)."""
 import os
 
@@ -91,66 +91,71 @@ def test_llama_micro_golden_logits(orc, name):
     assert np.array_equal(bits(m.eval(toks[13:15])), bits(z["logits_tail"]))
 
 
-# ---- live against the reference's compiled ggml.c (skips only if oracle/_ref is absent AND cannot be built) ----
+# ---- against the reference's compiled ggml.c (tests/golden/reference_outputs.json) ----
 
-def test_fp16_conversions_vs_reference(orc, ref):
+def fp16_inputs():
     rng = np.random.default_rng(7)
     xs = np.concatenate([rng.standard_normal(4000).astype(np.float32) * s for s in (1e-8, 1e-6, 1e-4, 1, 300, 7e4)] +
                         [np.array([0, -0.0, 65504, 65519.9, 65520, 1e-7, 5.96e-8, 2.98e-8, 3e-8, np.inf, -np.inf], np.float32)])
-    for x in xs:
-        assert ref.lib.rh_fp32_to_fp16(float(x)) == orc.lib.or_fp32_to_fp16(float(x)), x
-    for h in range(65536):
-        if (h & 0x7c00) != 0x7c00:
-            assert np.float32(ref.lib.rh_fp16_to_fp32(h)).tobytes() == np.float32(orc.lib.or_fp16_to_fp32(h)).tobytes(), h
+    hs = np.array([h for h in range(65536) if (h & 0x7c00) != 0x7c00], np.uint16)
+    return xs, hs
+
+
+def test_fp16_conversions_vs_reference(orc, reference):
+    xs, hs = fp16_inputs()
+    reference("fp16/fp32_to_fp16", np.array([orc.lib.or_fp32_to_fp16(float(x)) for x in xs], np.uint16))
+    reference("fp16/fp16_to_fp32", np.array([orc.lib.or_fp16_to_fp32(int(h)) for h in hs], np.float32))
+
+
+def rows_inputs(t, K):
+    rng = np.random.default_rng(K + t)
+    w = (rng.standard_normal((16, K)) / np.sqrt(K)).astype(np.float32)
+    x = (rng.standard_normal((3, K)) * rng.uniform(0.01, 30)).astype(np.float32)
+    return w, x
 
 
 @pytest.mark.parametrize("name,t", TYPES)
 @pytest.mark.parametrize("K", [64, 4096, 11008])
-def test_rows_vs_reference(orc, ref, name, t, K):
-    rng = np.random.default_rng(K + t)
-    w = (rng.standard_normal((16, K)) / np.sqrt(K)).astype(np.float32)
-    x = (rng.standard_normal((3, K)) * rng.uniform(0.01, 30)).astype(np.float32)
-    wq = ref.quantize(t, w)
-    assert np.array_equal(wq, orc.quantize(t, w))
-    vt = B.VEC_DOT_TYPE[t]
-    assert np.array_equal(ref.from_float(vt, x[0]), orc.from_float(vt, x[0]))
-    assert np.array_equal(bits(ref.mul_mat(t, wq, x, n_threads=3)), bits(orc.mul_mat(t, wq, x)))
+def test_rows_vs_reference(orc, reference, name, t, K):
+    w, x = rows_inputs(t, K)
+    wq = orc.quantize(t, w)
+    reference(f"rows/{name}/K{K}/quantize", wq)
+    reference(f"rows/{name}/K{K}/from_float", orc.from_float(B.VEC_DOT_TYPE[t], x[0]))
+    reference(f"rows/{name}/K{K}/mul_mat", orc.mul_mat(t, wq, x))
 
 
-@pytest.mark.parametrize("cfg,name", [("tiny", "q4_0"), ("tiny", "q4_1"), ("tiny", "q5_0"), ("small", "q5_1"), ("small", "q8_0")])
-def test_llama_vs_reference(orc, ref, cfg, name):
-    t = B.QUANT_TYPES[name]
-    hp, tens = synth.make_llama(synth.CONFIGS[cfg], t, orc.quantize)
+LLAMA_CASES = [("tiny", "q4_0"), ("tiny", "q4_1"), ("tiny", "q5_0"), ("small", "q5_1"), ("small", "q8_0")]
+
+
+@pytest.mark.parametrize("cfg,name", LLAMA_CASES)
+def test_llama_vs_reference(orc, reference, cfg, name):
+    hp, tens = synth.make_llama(synth.CONFIGS[cfg], B.QUANT_TYPES[name], orc.quantize)
     toks = synth.make_tokens(hp, 37)
-    mr = ref.llama(hp, tens, n_threads=4, n_batch=64)
     mo = orc.llama(hp, tens)
-    assert np.array_equal(bits(mr.eval(toks[:33])), bits(mo.eval(toks[:33])))
-    assert np.array_equal(bits(mr.eval(toks[33:34])), bits(mo.eval(toks[33:34])))
-    assert np.array_equal(bits(mr.eval(toks[34:37])), bits(mo.eval(toks[34:37])))
-    assert np.array_equal(mr.kv(0), mo.kv(0)) and np.array_equal(mr.kv(1), mo.kv(1))
-    # the reference result does not depend on the thread split nor on batching (one vec_dot per dst element)
-    mr1 = ref.llama(hp, tens, n_threads=1, n_batch=64)
-    rows = np.concatenate([mr1.eval(toks[i:i + 1]) for i in range(8)])
+    key = f"llama/{cfg}/{name}"
+    for lo, hi in ((0, 33), (33, 34), (34, 37)):
+        reference(f"{key}/eval {lo}:{hi}", mo.eval(toks[lo:hi]))
+    reference(f"{key}/kv 0", mo.kv(0))
+    reference(f"{key}/kv 1", mo.kv(1))
+    # the reference result does not depend on the thread split nor on batching (one vec_dot per dst element): the recorded rows are its
+    # single-threaded token-by-token evaluation
     mo.reset()
-    assert np.array_equal(bits(rows), bits(mo.eval(toks[:8])))
+    reference(f"{key}/token by token 0:8", mo.eval(toks[:8]))
 
 
-def test_llama_rope_overrides_and_set_n_past_vs_reference(orc, ref):
+def test_llama_rope_overrides_and_set_n_past_vs_reference(orc, reference):
     """RoPEOverrides (op_rope_inplace -> ggml_rope_custom_inplace, crates/ggml/src/context.rs:558-590) and the position restore used
     by bench.py's CPU arm: the plain-C port and the reference's compiled ggml.c agree bit for bit."""
     hp, tens = synth.make_llama(synth.CONFIGS["tiny"], B.Q4_0, orc.quantize)
     toks = synth.make_tokens(hp, 30)
-    mr = ref.llama(hp, tens, n_threads=3, n_batch=64)
     mo = orc.llama(hp, tens)
     plain = mo.eval(toks[:9]).copy()
     mo.reset()
-    for m in (mr, mo):
-        m.set_rope(26000.0, 0.5)
-    a, b = mr.eval(toks[:20]), mo.eval(toks[:20])
-    assert np.array_equal(bits(a), bits(b))
+    mo.set_rope(26000.0, 0.5)
+    b = mo.eval(toks[:20])
+    reference("rope_overrides/eval 0:20", b)
     assert not np.array_equal(bits(b[:9]), bits(plain))                 # the override really changes the result
-    assert np.array_equal(bits(mr.eval(toks[20:21])), bits(mo.eval(toks[20:21])))
-    # rewind both to position 12 (the cache rows 12.. are simply overwritten) and continue
-    for m in (mr, mo):
-        m.set_n_past(12)
-    assert np.array_equal(bits(mr.eval(toks[12:15])), bits(mo.eval(toks[12:15])))
+    reference("rope_overrides/eval 20:21", mo.eval(toks[20:21]))
+    # rewind to position 12 (the cache rows 12.. are simply overwritten) and continue
+    mo.set_n_past(12)
+    reference("rope_overrides/eval 12:15 after set_n_past(12)", mo.eval(toks[12:15]))
