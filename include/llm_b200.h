@@ -151,7 +151,7 @@ int  b200_session_sync(b200_session *s);
 /* with B200_DECODE_PROF=1 in the environment the decode kernel stamps %globaltimer (ns) at its phase boundaries (CTA 0);
  * slot 0 = start, then pairs (before / after grid barrier) per phase in graph order, slot 127 = end of token */
 int  b200_session_decode_profile(b200_session *s, unsigned long long *out128);
-/* tuning aid (B200_DECODE_PROF=1): per-launch %globaltimer stamps of the graph decode schedule; out = 8*n values, see session.cu */
+/* tuning aid (B200_DECODE_PROF=1): per-launch %globaltimer stamps of the graph decode schedule; out = 9*n values, see session.cu */
 int  b200_session_decode_timeline(b200_session *s, unsigned long long *out, int n, int reset);
 /* debug taps for parity work: keep a copy of one intermediate buffer of (layer, stage) during the next evaluate.
  * stages: 1 attn-norm out [n][e], 2 qkv before rope [n][e+2gqa], 3 qkv after rope, 4 KQ raw [h][n][n_kv], 5 KQ softmax, 6 merged

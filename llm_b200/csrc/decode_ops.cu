@@ -33,8 +33,13 @@ __constant__ TpCtx c_tp;
 
 namespace {
 
-// Programmatic dependent launch.  Every kernel of the chain touches nothing a predecessor writes (and writes nothing at all) before
-// `pdl_wait`; what runs ahead of the wait only reads the constant weights (the producer warp of the next mat-vec fills its ring).
+// Programmatic dependent launch.  Every kernel of the chain touches nothing a predecessor of the same token writes (and writes nothing at
+// all) before `pdl_wait`.  What runs ahead of the wait reads the constant weights (the producer warp of the next mat-vec fills its ring)
+// and, in the fused attention, n_past and the layer's K rows / V columns below n_past: within one token n_past changes only in the last
+// node (EPI_LOGITS, EPI_BIAS with n_past_inc), which starts after every attention launch has completed, and the only writer of a layer's
+// cache is the launch right before its attention (mmv<EPI_QKV>, or neox_rope_store_kernel for GPT-NeoX / GPT-2), which writes K row and
+// V column n_past and nothing else.  Everything below n_past was written by earlier tokens or batches, which are stream-ordered before
+// this token's graph (its first node is an ordinary launch).  Tensor-parallel ranks hold their own heads of the cache: the same holds.
 // WHERE the dependents are released matters (B200, LLaMA-7B decode, ms/token): trigger at kernel entry 2.41 (the successors sit on SM
 // resources the running kernel's tail needs), no PDL 1.757, trigger after the last tile is consumed 1.729, trigger from the producer warp
 // as soon as every byte of the CTA is requested 1.705 -> that is the default.
@@ -43,6 +48,10 @@ __device__ __forceinline__ unsigned long long gtime() { unsigned long long t; as
 __device__ __forceinline__ void prof_begin(unsigned long long *p) { if (p && threadIdx.x == 0) { const unsigned long long t = gtime(); atomicMin(p, t); atomicMax(p + 3 * B200_PROF_SLOTS, t); } }
 __device__ __forceinline__ void prof_ready(unsigned long long *p) { if (p && threadIdx.x == 0) { const unsigned long long t = gtime(); atomicMin(p + 2 * B200_PROF_SLOTS, t); atomicMax(p + 4 * B200_PROF_SLOTS, t); } }
 __device__ __forceinline__ void prof_end(unsigned long long *p) { if (p && threadIdx.x == 0) atomicMax(p + B200_PROF_SLOTS, gtime()); }
+// a phase boundary: earliest CTA into array kmin (one that holds minima, or -1 for none), latest into array kmax
+__device__ __forceinline__ void prof_stamp(unsigned long long *p, int kmin, int kmax) {
+    if (p && threadIdx.x == 0) { const unsigned long long t = gtime(); if (kmin >= 0) atomicMin(p + kmin * B200_PROF_SLOTS, t); atomicMax(p + kmax * B200_PROF_SLOTS, t); }
+}
 
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -52,6 +61,12 @@ int pdl_mask() {
     static int mask = -1;
     if (mask < 0) { const char *e = getenv("B200_PDL"); mask = e ? atoi(e) : 3; }
     return mask;
+}
+// B200_ATTN_PREFETCH: 1 (default) = the fused attention streams the cached K/V below n_past ahead of its pdl_wait, 0 = every load after it
+int attn_prefetch() {
+    static int on = -1;
+    if (on < 0) { const char *e = getenv("B200_ATTN_PREFETCH"); on = e ? (atoi(e) != 0) : 1; }
+    return on;
 }
 
 template <int CLASS = 2, typename... KArgs, typename... Args>
@@ -453,7 +468,7 @@ template <bool TP>
 __global__ void __launch_bounds__(ATH) attn_fused_kernel(const float *__restrict__ q, const __half *__restrict__ Kl, const __half *__restrict__ Vl,
                                                          int4 *__restrict__ xpack_out, const int *__restrict__ n_past, const uint16_t *__restrict__ lut_exp,
                                                          float kq_scale, int hd, int n_head, int n_head_kv, int gqa, int n_ctx, int nlay, int q81, int off, int scale16,
-                                                         unsigned long long *prof, const TpSync S, int head0) {
+                                                         unsigned long long *prof, const TpSync S, int head0, int prefetch) {
     const TpCtx &T = c_tp;
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
@@ -472,53 +487,78 @@ __global__ void __launch_bounds__(ATH) attn_fused_kernel(const float *__restrict
     __half *q16 = p16 + nlay;
     __half *vs = (__half *)(sm + (((size_t)nlay * 6 + (size_t)hd * 2 + 127) & ~(size_t)127));
     pdl_trigger();                                              // the successor (wo) only needs shared memory beside us: let it prefetch its tiles now
-    pdl_wait();
-    float qv = 0.f;
-    if (tid < hd) qv = __ldcg(q + h * hd + tid);               // in flight together with the n_past load (hd <= 256 = ATH)
-    const int n_kv = __ldcg(n_past) + 1;
+    if (!prefetch) { pdl_wait(); prof_ready(prof); }
+    // With `prefetch`, everything up to the pdl_wait below runs while the QKV launch is still finishing: it reads only what that launch does
+    // not write (the rule at the top of this file).  The K row and the V column at n_past are the QKV launch's output: loaded after the wait.
+    const int n_kv = __ldcg(n_past) + 1, p = n_kv - 1;
     const int np = n_kv & ~31;
 
-    {   // V rows of this CTA's 32 channels: all copies in flight now, consumed after the soft_max
-        const int cpr = (n_kv + 7) / 8;                          // 16-byte chunks per row
-        for (int i = tid; i < 32 * cpr; i += ATH) {
-            const int rr = i / cpr, cc = i - rr * cpr;
+    // V rows of this CTA's 32 channels: all copies in flight at once, consumed after the soft_max
+    const int cpr = (n_kv + 7) / 8;                              // 16-byte chunks per row
+    auto copy_v = [&](int c_lo, int c_hi) {
+        const int nc = c_hi - c_lo;
+        for (int i = tid; i < 32 * nc; i += ATH) {
+            const int rr = i / nc, cc = c_lo + i - rr * nc;
             cp16(smem_u32(vs + rr * vstride + cc * 8), Vl + (int64_t)(hk * hd + c0 + rr) * n_ctx + cc * 8);
         }
-    }
-    if (tid < hd) q16[tid] = __float2half_rn(qv);
-    // q16 visible inside the CTA; every CTA of the cluster is running before its shared memory is written remotely (no data is exchanged
-    // yet, so the cluster barrier can be the relaxed one: no fence)
-    __syncthreads();
-    asm volatile("barrier.cluster.arrive.relaxed.aligned;\n\tbarrier.cluster.wait.aligned;" ::: "memory");
+    };
+    const int vpre = prefetch ? p / 8 : 0;                       // chunks that lie entirely below column n_past
 
-    // ---- KQ for this CTA's share of the positions ----
-    {
-        const int per = (n_kv + per_head - 1) / per_head, j0 = part * per, j1 = n_kv < j0 + per ? n_kv : j0 + per;
-        const int nvec = hd / 32;                                // 16-byte loads per thread per position (chunks i = 0..nvec-1)
-        constexpr int PU = 4;                                    // positions per quad per pass: up to 4 * nvec 16-byte loads in flight per thread
-        for (int jb = j0; jb < j1; jb += PU * (ATH / 4)) {
-            int4 kv[PU][4];
+    // KQ for this CTA's share [j0, j1) of the positions, one pass = PU positions per quad; pass 0's K rows below n_past are loaded now
+    const int per = (n_kv + per_head - 1) / per_head, j0 = part * per, j1 = n_kv < j0 + per ? n_kv : j0 + per;
+    const int nvec = hd / 32;                                    // 16-byte loads per thread per position (chunks i = 0..nvec-1)
+    constexpr int PU = 4;                                        // positions per quad per pass: up to 4 * nvec 16-byte loads in flight per thread
+    int4 kv[PU][4];
+    auto load_k = [&](int jb, int jend) {                        // rows j < jend (<= j1) of the pass at jb, zeros from there on
 #pragma unroll
-            for (int pu = 0; pu < PU; pu++) {
-                const int j = jb + pu * (ATH / 4) + (tid >> 2);
-                const __half *krow = Kl + (int64_t)(j < j1 ? j : j0) * gqa + hk * hd + 8 * u;
+        for (int pu = 0; pu < PU; pu++) {
+            const int j = jb + pu * (ATH / 4) + (tid >> 2);
+            const __half *krow = Kl + (int64_t)(j < jend ? j : j0) * gqa + hk * hd + 8 * u;
 #pragma unroll
-                for (int i = 0; i < 4; i++) if (i < nvec) kv[pu][i] = j < j1 ? __ldcg((const int4 *)(krow + 32 * i)) : make_int4(0, 0, 0, 0);
+            for (int i = 0; i < 4; i++) if (i < nvec) kv[pu][i] = j < jend ? __ldcg((const int4 *)(krow + 32 * i)) : make_int4(0, 0, 0, 0);
+        }
+    };
+    // K first: the scores need it long before KQV needs V, and loads issued behind the V burst queue behind it
+    load_k(j0, prefetch ? (p < j1 ? p : j1) : 0);
+    copy_v(0, vpre);
+    // every CTA of the cluster is running before its shared memory is written remotely (no data is exchanged yet, so the cluster barrier
+    // can be the relaxed one: no fence)
+    asm volatile("barrier.cluster.arrive.relaxed.aligned;\n\tbarrier.cluster.wait.aligned;" ::: "memory");
+    if (prefetch) { pdl_wait(); prof_ready(prof); }
+
+    float qv = 0.f;
+    if (tid < hd) qv = __ldcg(q + h * hd + tid);               // hd <= 256 = ATH
+    if (!prefetch) load_k(j0, j1);
+    else {                                                       // row n_past, if it lies in pass 0 (past j1 too: that score is not stored, and
+#pragma unroll                                                   // the guard would cost 16 registers)
+        for (int pu = 0; pu < PU; pu++)
+            if (j0 + pu * (ATH / 4) + (tid >> 2) == p) {
+                const __half *krow = Kl + (int64_t)p * gqa + hk * hd + 8 * u;
+#pragma unroll
+                for (int i = 0; i < 4; i++) if (i < nvec) kv[pu][i] = __ldcg((const int4 *)(krow + 32 * i));
             }
+    }
+    copy_v(vpre, cpr);
+    if (tid < hd) q16[tid] = __float2half_rn(qv);
+    __syncthreads();                                             // q16 visible inside the CTA
+
+    for (int jb = j0; jb < j1; jb += PU * (ATH / 4)) {
+        if (jb != j0) load_k(jb, j1);
 #pragma unroll
-            for (int pu = 0; pu < PU; pu++) {
-                const int j = jb + pu * (ATH / 4) + (tid >> 2);
-                float acc[8];
+        for (int pu = 0; pu < PU; pu++) {
+            const int j = jb + pu * (ATH / 4) + (tid >> 2);
+            float acc[8];
 #pragma unroll
-                for (int e = 0; e < 8; e++) acc[e] = 0.f;
+            for (int e = 0; e < 8; e++) acc[e] = 0.f;
 #pragma unroll
-                for (int i = 0; i < 4; i++) if (i < nvec) fma8(acc, kv[pu][i], *(const int4 *)(q16 + 32 * i + 8 * u));
-                const float s = quad_tree(acc);
-                if (j < j1 && u < per_head) cluster.map_shared_rank(sc, u)[j] = __fmul_rn(s, kq_scale);   // thread u of the quad feeds CTA u
-            }
+            for (int i = 0; i < 4; i++) if (i < nvec) fma8(acc, kv[pu][i], *(const int4 *)(q16 + 32 * i + 8 * u));
+            const float s = quad_tree(acc);
+            if (j < j1 && u < per_head) cluster.map_shared_rank(sc, u)[j] = __fmul_rn(s, kq_scale);   // thread u of the quad feeds CTA u
         }
     }
+    prof_stamp(prof, 5, 6);                                      // this CTA's K rows have landed and its scores are out
     cluster.sync();
+    prof_stamp(prof, -1, 7);
 
     // ---- soft_max over sc[0, n_kv) (ggml_compute_forward_soft_max_f32, LC/ggml.c:11700-11770: fp16 exp table, double row sum) ----
     float mx = -INFINITY;
@@ -543,6 +583,7 @@ __global__ void __launch_bounds__(ATH) attn_fused_kernel(const float *__restrict
     __syncthreads();
     const float inv = (float)(1.0 / (((shd[0] + shd[1]) + (shd[2] + shd[3])) + ((shd[4] + shd[5]) + (shd[6] + shd[7]))));
     for (int j = tid; j < n_kv; j += ATH) p16[j] = __float2half_rn(__fmul_rn(sc[j], inv));
+    prof_stamp(prof, -1, 8);
     asm volatile("cp.async.wait_all;" ::: "memory");
     __syncthreads();
 
@@ -695,7 +736,7 @@ void decode_ops_t(const DecodeParams &P, const std::vector<DecodeLayer> &layers,
             cfg.attrs = at; cfg.numAttrs = (pdl_mask() & 2) ? 2 : 1;
             B200_CHECK(cudaLaunchKernelEx(&cfg, attn_fused_kernel<TP>, (const float *)P.q, (const __half *)L.K, (const __half *)L.V, P.xpack_d, (const int *)P.n_past,
                                           (const uint16_t *)P.lut_exp, P.kq_scale, P.hd, P.n_head, P.n_head_kv, P.gqa, P.n_ctx, nlay, q81, off, s16, pr(),
-                                          ts(-1, 0, -1, 0, TPB_XD, v), tp ? P.head0 : 0));
+                                          ts(-1, 0, -1, 0, TPB_XD, v), tp ? P.head0 : 0, attn_prefetch()));
             n++;
         } else {
             launch_k(P.hd == 128 ? attn_kq_kernel<128> : attn_kq_kernel<64>, dim3((n_kv_bucket + 63) / 64, P.n_head), dim3(128), 0, st,
@@ -842,7 +883,7 @@ void neox_ops_t(const NeoxParams &P, const std::vector<NeoxLayer> &layers, int n
             cfg.attrs = at; cfg.numAttrs = (pdl_mask() & 2) ? 2 : 1;
             B200_CHECK(cudaLaunchKernelEx(&cfg, attn_fused_kernel<false>, (const float *)P.q, (const __half *)L.K, (const __half *)L.V, P.xpack_d, (const int *)P.n_past,
                                           (const uint16_t *)P.lut_exp, P.kq_scale, P.hd, P.n_head, P.n_head, e, P.n_ctx, nlay, q81, off, s16,
-                                          (unsigned long long *)nullptr, S, 0));                                                           // :250-298
+                                          (unsigned long long *)nullptr, S, 0, attn_prefetch()));                                                           // :250-298
             n++;
         }
         // attention.dense (+bias); sequential residual: ff_in = that + inpL                                                                    :301-312

@@ -550,8 +550,8 @@ static b200_session *start_session_tp(b200_session *s) {
     B200_CHECK(cudaMalloc(&s->xpack_a, (e / QK) * 64));
     B200_CHECK(cudaMalloc(&s->d_n_past, sizeof(int)));
     B200_CHECK(cudaMallocHost(&s->h_n_past, sizeof(int)));
-    B200_CHECK(cudaMalloc(&s->d_prof, B200_PROF_SLOTS * 8 * sizeof(unsigned long long)));
-    B200_CHECK(cudaMemset(s->d_prof, 0, B200_PROF_SLOTS * 8 * sizeof(unsigned long long)));
+    B200_CHECK(cudaMalloc(&s->d_prof, B200_PROF_SLOTS * 9 * sizeof(unsigned long long)));
+    B200_CHECK(cudaMemset(s->d_prof, 0, B200_PROF_SLOTS * 9 * sizeof(unsigned long long)));
     // the exchange slab: arrays of 8-byte {word, tag} units (tp.cuh) -- x | ff | attention records | ffn records | logits, 256-byte aligned pieces
     TpCtx &T = s->dp.tp;
     T = TpCtx();
@@ -667,8 +667,8 @@ b200_session *b200_model_start_session(b200_model *m, const b200_session_config 
     P.xpack_d = s->xpack_d; P.xpack_f = s->xpack_f;
     B200_CHECK(cudaMalloc(&s->xpack_a, (e / QK) * 64));
     P.scratch_bytes = decode_scratch_bytes((int)e, (int)f, m->hd, (int)n_ctx);
-    B200_CHECK(cudaMalloc(&s->d_prof, B200_PROF_SLOTS * 8 * sizeof(unsigned long long)));
-    B200_CHECK(cudaMemset(s->d_prof, 0, B200_PROF_SLOTS * 8 * sizeof(unsigned long long)));
+    B200_CHECK(cudaMalloc(&s->d_prof, B200_PROF_SLOTS * 9 * sizeof(unsigned long long)));
+    B200_CHECK(cudaMemset(s->d_prof, 0, B200_PROF_SLOTS * 9 * sizeof(unsigned long long)));
     P.prof = getenv("B200_DECODE_PROF") ? s->d_prof : nullptr;
     s->mega_ok = hp.n_rot == m->hd && (m->hd == 64 || m->hd == 128) && decode_supported(P, hp.wtype);
     B200_CHECK(cudaDeviceSynchronize());   // the memsets / copies above ran on the legacy stream: order them before anything on the backend's non-blocking stream
@@ -782,17 +782,19 @@ int b200_session_decode_profile(b200_session *s, unsigned long long *out128) {
 }
 
 // Per-kernel timeline of the graph decode schedule (B200_DECODE_PROF=1): slot i = the i-th launch of the token;
-// out = 8 arrays of n (%globaltimer, ns): CTA begin min, CTA end max, prologue-done min, begin max, prologue-done max, first stage landed min / max,
-// last stage landed max (mat-vec kernels only for the last three).  reset != 0 re-arms the slots.
+// out = 9 arrays of n (%globaltimer, ns): CTA begin min, CTA end max, prologue-done min, begin max, prologue-done max, first stage landed min / max,
+// last stage landed max (mat-vec kernels only for the last three), unused by the mat-vecs.  The fused attention stamps its phases into arrays
+// 2 / 4 (past pdl_wait, first / last CTA), 5 / 6 (KQ share done), 7 (scores exchanged, last CTA) and 8 (soft_max done, last CTA).
+// reset != 0 re-arms the slots.
 int b200_session_decode_timeline(b200_session *s, unsigned long long *out, int n, int reset) {
     if (!s || n < 0 || n > B200_PROF_SLOTS) return B200_ERR_BAD_ARG;
     B200_CHECK(cudaStreamSynchronize(rt().stream));
     if (out && n) {
-        for (int k = 0; k < 8; k++)
+        for (int k = 0; k < 9; k++)
             B200_CHECK(cudaMemcpy(out + (size_t)k * n, s->d_prof + (size_t)k * B200_PROF_SLOTS, (size_t)n * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     }
     if (reset) {                                                  // arrays 0, 2, 5 hold minima, the others maxima
-        for (int k = 0; k < 8; k++)
+        for (int k = 0; k < 9; k++)
             B200_CHECK(cudaMemset(s->d_prof + (size_t)k * B200_PROF_SLOTS, (k == 0 || k == 2 || k == 5) ? 0xFF : 0, B200_PROF_SLOTS * sizeof(unsigned long long)));
         B200_CHECK(cudaDeviceSynchronize());
     }

@@ -20,10 +20,10 @@ per_layer = ["norm", "qkv", "attn", "wo", "norm2", "w13", "w2"] if os.environ.ge
 n = len(per_layer) * nl + 3
 L.b200_session_decode_timeline(s._s, None, 0, 1)
 s.evaluate(toks[517:518])
-buf = (C.c_ulonglong * (8 * n))()
+buf = (C.c_ulonglong * (9 * n))()
 L.b200_session_decode_timeline(s._s, buf, n, 0)
-t = np.array(buf[:], dtype=np.float64).reshape(8, n)
-beg, end, rdy, begx, rdyx, ff, ffx, lf = t
+t = np.array(buf[:], dtype=np.float64).reshape(9, n)
+beg, end, rdy, begx, rdyx, ff, ffx, lf, sm = t
 names = ["embed"] + per_layer * nl + ["normF", "logits"]
 t0 = beg[1]
 print("token span %.1f us (first norm begin -> logits end)" % ((end[-1] - t0) / 1e3))
@@ -44,3 +44,11 @@ for k, a in agg.items():
     print(f"  {k:7s} n={c:3d} dur {v[0]:6.2f} gap {v[1]:5.2f} | lastCTA {v[2]:5.2f} | xready {v[3]:5.2f}/{v[4]:5.2f} | stage0 {v[5]:5.2f}/{v[6]:5.2f} | laststage {v[7]:6.2f} | total {(a[1]+a[2])/1e3:6.3f} ms")
     tot_d += a[1]; tot_g += a[2]
 print(f"sum durations {tot_d/1e3:.3f} ms, sum gaps {tot_g/1e3:.3f} ms")
+# the fused attention's phases (decode_ops.cu attn_fused_kernel), mean us relative to the first CTA's start; the QKV launch before it is the
+# one its pdl_wait waits for
+ia = [i for i in range(1, n) if names[i] == "attn"]
+if ia:
+    m = lambda a, idx=None: float(np.nanmean([rel(a, i) if idx is None else (a[idx(i)] - beg[i]) / 1e3 for i in ia]))
+    print("attn phases, mean us relative to the first CTA's start (first/last CTA):")
+    print(f"  lastCTA start {m(begx):5.2f} | qkv end {m(end, lambda i: i - 1):5.2f} | past pdl_wait {m(rdy):5.2f}/{m(rdyx):5.2f} | "
+          f"KQ share done {m(ff):5.2f}/{m(ffx):5.2f} | scores exchanged {m(lf):5.2f} | soft_max done {m(sm):5.2f} | end {m(end):5.2f}")
