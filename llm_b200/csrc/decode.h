@@ -68,6 +68,11 @@ bool decode_supported(const DecodeParams &P, int wtype);
 // cooperative launch on `st`; returns false if the kernel cannot be made resident (caller falls back to the per-op schedule)
 bool launch_decode(const DecodeParams &P, int wtype, cudaStream_t st, int *grid_out);
 
+// whether the cluster attention kernel of the fused decode schedules (decode_ops.cu) holds a context bucket of n_kv_bucket positions in shared
+// memory at head size hd: true up to a bucket of 3072 (and for a last bucket, capped at n_ctx, of up to 3264).  LLaMA decodes the larger buckets
+// through the two-kernel attention, GPT-NeoX / GPT-2 through the per-op schedule; a tensor-parallel session needs every bucket to fit.
+bool attn_fused_fits(int n_kv_bucket, int hd);
+
 // default decode schedule: 8 fused kernels per layer on `st` (decode_ops.cu); position read from *P.n_past on the device
 void decode_ops_enqueue(const DecodeParams &P, const std::vector<DecodeLayer> &layers, int wtype, int n_kv_bucket, int4 *xpack_a, cudaStream_t st, int *launches);
 

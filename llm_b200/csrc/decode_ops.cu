@@ -4,7 +4,7 @@
 //   2 mmv<QKV>         [wq|wk|wv] x, epilogue: RoPE on Q/K rows, K/V rows -> f16 cache at n_past (:190-244)
 //   3 attn_fused       KQ = K . f16(Q), scale + soft_max, V^T . f16(P), epilogue: quantize the merged row -- one cluster of hd/32 CTAs per
 //                      head, scores exchanged through distributed shared memory                (:246-307)
-//                      (B200_ATTN_FUSED=0: the two-kernel variant attn_kq + attn_sv)
+//                      (B200_ATTN_FUSED=0, and context buckets past 3072 positions: the two-kernel variant attn_kq + attn_sv)
 //   4 mmv<RES>         wo x + inpSA                                                           (:310-314)
 //   5 norm_pack        rms_norm(inpFF) * ffn_norm                                             (:318-321)
 //   6 mmv<SILU>        [w1|w3] x (rows interleaved in 32-row pieces), epilogue: silu(w1 x) * (w3 x) quantized (:323-330)
@@ -653,6 +653,13 @@ void launch_mmv(const QWeight &w, MmvArgs A, cudaStream_t st) {
     launch_k<1>(mmv_fused_kernel<TYPE, EPI, TP>, dim3((unsigned)(groups < slots ? groups : slots)), dim3(STHREADS), (size_t)smem_of(nst), st, w, A);
 }
 
+// dynamic shared memory of the cluster attention kernel for a context bucket (attn_fused_kernel's layout): f32 scores, f16 probabilities and q16,
+// rounded to 128 B, then 32 staged V rows of nlay + 32 halves
+size_t attn_fused_smem(int n_kv_bucket, int hd) {
+    const size_t nlay = (size_t)(n_kv_bucket + 63) / 64 * 64;
+    return ((nlay * 6 + (size_t)hd * 2 + 127) & ~(size_t)127) + (size_t)32 * (nlay + 32) * 2;
+}
+
 // dynamic shared memory opt-in of the cluster attention kernel: one high-water mark for both instantiations (the attribute is per function, not per caller)
 static void attn_fused_reserve(size_t bytes) {
     static size_t set = 48 * 1024;
@@ -708,12 +715,14 @@ void decode_ops_t(const DecodeParams &P, const std::vector<DecodeLayer> &layers,
     };
     get_rows_q(P.wte, P.token, P.x, 1, st); n++;
     if (tp) { launch_k(tp_spread_kernel, dim3((e + 255) / 256), dim3(256), 0, st, (const float *)P.x, e); n++; }
-    // attention: one cluster launch per layer (default) or the two-kernel variant (B200_ATTN_FUSED=0, or head sizes a cluster cannot cover)
+    // attention: one cluster launch per layer (default) or the two-kernel variant (B200_ATTN_FUSED=0, head sizes a cluster cannot cover, or a
+    // context bucket whose scores and V rows do not fit one CTA's shared memory: past 3072 positions)
     static const bool fused_env = !(getenv("B200_ATTN_FUSED") && getenv("B200_ATTN_FUSED")[0] == '0');
     const int nlay = (n_kv_bucket + 63) / 64 * 64;
-    const size_t fa_smem = (((size_t)nlay * 6 + (size_t)P.hd * 2 + 127) & ~(size_t)127) + (size_t)32 * (nlay + 32) * 2;
-    const bool fused_attn = (fused_env || tp) && P.hd % 32 == 0 && P.hd <= 128 && P.n_ctx % 8 == 0 && fa_smem <= 227 * 1024;
-    B200_ASSERT(fused_attn || !tp);                              // the tensor-parallel exchange lives in the fused attention kernel's epilogue
+    const size_t fa_smem = attn_fused_smem(n_kv_bucket, P.hd);
+    const bool fused_attn = (fused_env || tp) && P.hd % 32 == 0 && P.hd <= 128 && P.n_ctx % 8 == 0 && attn_fused_fits(n_kv_bucket, P.hd);
+    // the tensor-parallel exchange lives in the fused attention kernel's epilogue; start_session_tp refuses a context whose buckets do not all fit
+    B200_ASSERT(fused_attn || !tp);
     if (fused_attn) attn_fused_reserve(fa_smem);
     const size_t sv_smem = (size_t)P.n_ctx * 6 + 32 * KC * 2 + 32 * 32 * 2;
     static size_t sv_set = 48 * 1024;
@@ -860,8 +869,9 @@ void neox_ops_t(const NeoxParams &P, const std::vector<NeoxLayer> &layers, int n
     get_rows_q(P.wte, P.token, P.x, 1, st); n++;
     if (P.wpe) { launch_k(gpt2_add_pos_kernel, dim3((e + 255) / 256), dim3(256), 0, st, P.x, P.wpe, (const int *)P.n_past, e); n++; }
     const int nlay = (n_kv_bucket + 63) / 64 * 64;
-    const size_t fa_smem = (((size_t)nlay * 6 + (size_t)P.hd * 2 + 127) & ~(size_t)127) + (size_t)32 * (nlay + 32) * 2;
-    B200_ASSERT(P.hd % 32 == 0 && P.hd <= 128 && P.n_ctx % 8 == 0 && fa_smem <= 227 * 1024 && e <= 8192);
+    const size_t fa_smem = attn_fused_smem(n_kv_bucket, P.hd);
+    // neox.cu decodes a token whose bucket does not fit through the per-op schedule instead
+    B200_ASSERT(P.hd % 32 == 0 && P.hd <= 128 && P.n_ctx % 8 == 0 && attn_fused_fits(n_kv_bucket, P.hd) && e <= 8192);
     attn_fused_reserve(fa_smem);
     const dim3 ln_grid((e / 4 + 255) / 256);
     const TpSync S{};
@@ -905,6 +915,8 @@ void neox_ops_t(const NeoxParams &P, const std::vector<NeoxLayer> &layers, int n
 }
 
 }  // namespace
+
+bool attn_fused_fits(int n_kv_bucket, int hd) { return attn_fused_smem(n_kv_bucket, hd) <= 227 * 1024; }
 
 void neox_decode_enqueue(const NeoxParams &P, const std::vector<NeoxLayer> &layers, int wtype, int n_kv_bucket, cudaStream_t st, int *launches) {
     switch (wtype) {

@@ -7,7 +7,8 @@
 //           InferenceSession::compute           crates/llm-base/src/inference_session.rs:114-295
 // Batches (prefill) run node by node on the bit-exact kernels of this directory (LayerNorm, bias adds, RoPE mode 2 on n_rot of the head size, gelu table,
 // exact quantized mat-muls incl. the tcgen05 GEMM, exact f16 attention mat-muls); single tokens run the fused 8-kernels-per-layer schedule of
-// decode_ops.cu::neox_decode_enqueue from one CUDA graph per context bucket.  Logits are bit-identical to the reference's CPU path (tests/test_gpu_neox.py).
+// decode_ops.cu::neox_decode_enqueue from one CUDA graph per context bucket, up to the largest bucket its attention holds (attn_fused_fits: 3072
+// positions), and node by node past it.  Logits are bit-identical to the reference's CPU path (tests/test_gpu_neox.py, tests/test_gpu_long_context.py).
 #include <string.h>
 
 #include <string>
@@ -129,13 +130,14 @@ void forward(b200_neox_session *s, int n, bool all_rows) {
     cudaStream_t st = rt().stream;
     const int e = hp.n_embd, hd = m->hd, n_head = hp.n_head, n_ctx = hp.context_size, n_past = s->n_past, n_kv = n_past + n;
     int L = 0;
-    if (n == 1 && s->decode_ok) {
+    int bucket = ((n_kv + 255) / 256) * 256; if (bucket > n_ctx) bucket = n_ctx;
+    // a bucket the cluster attention cannot hold (past 3072 positions) decodes through the per-op schedule below, which leaves d_n_past alone
+    if (n == 1 && s->decode_ok && attn_fused_fits(bucket, hd)) {
         if (s->dev_n_past != n_past) {
             B200_CHECK(cudaStreamSynchronize(st));
             *s->h_n_past = n_past;
             B200_CHECK(cudaMemcpyAsync(s->d_n_past, s->h_n_past, sizeof(int), cudaMemcpyHostToDevice, st));
         }
-        int bucket = ((n_kv + 255) / 256) * 256; if (bucket > n_ctx) bucket = n_ctx;
         int nodes = 0;
         if (!s->decode_warm) {
             neox_decode_enqueue(s->dp, s->dl, hp.wtype, bucket, st, &nodes);

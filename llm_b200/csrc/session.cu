@@ -88,8 +88,9 @@ struct b200_session {
     std::vector<DecodeLayer> h_layers;                 // host copy of the layer table (kernel arguments of the decode graph)
     int4 *xpack_a = nullptr;
     bool decode_warm = false;                          // first decode step runs eagerly (sets kernel attributes), later ones replay a graph
-    std::vector<std::pair<int, cudaGraphExec_t>> graphs;   // (n_kv bucket, instantiated graph)
-    int graph_nodes = 0;
+    // instantiated decode graph per n_kv bucket, with its kernel count: buckets past 3072 positions run the two-kernel attention (one more per layer)
+    struct DecodeGraph { int bucket; cudaGraphExec_t exec; int nodes; };
+    std::vector<DecodeGraph> graphs;
     DecodeParams dp;
     int tap_layer = -2, tap_stage = 0;
     float *tap = nullptr; size_t tap_cap = 0, tap_count = 0;
@@ -205,24 +206,26 @@ void forward(b200_session *s, int n, bool all_rows = true) {
             int nodes = 0;
             if (!s->decode_warm || (s->cfg.flags & B200_SESSION_NO_GRAPH)) {
                 decode_ops_enqueue(s->dp, s->h_layers, hp.wtype, bucket, s->xpack_a, st, &nodes);
-                s->decode_warm = true; s->graph_nodes = nodes;
+                s->decode_warm = true;
             } else {
-                cudaGraphExec_t exec = nullptr;
-                for (auto &g : s->graphs) if (g.first == bucket) exec = g.second;
-                if (!exec) {
+                const b200_session::DecodeGraph *g = nullptr;
+                for (auto &c : s->graphs) if (c.bucket == bucket) g = &c;
+                if (!g) {
                     cudaGraph_t graph;
+                    cudaGraphExec_t exec;
                     B200_CHECK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
                     decode_ops_enqueue(s->dp, s->h_layers, hp.wtype, bucket, s->xpack_a, st, &nodes);
                     B200_CHECK(cudaStreamEndCapture(st, &graph));
                     B200_CHECK(cudaGraphInstantiate(&exec, graph, 0));
                     B200_CHECK(cudaGraphDestroy(graph));
-                    s->graphs.emplace_back(bucket, exec);
-                    s->graph_nodes = nodes;
+                    s->graphs.push_back({bucket, exec, nodes});
+                    g = &s->graphs.back();
                 }
-                B200_CHECK(cudaGraphLaunch(exec, st));
+                nodes = g->nodes;
+                B200_CHECK(cudaGraphLaunch(g->exec, st));
             }
             s->dev_n_past = n_past + 1;
-            s->last_launches = s->graph_nodes; s->last_n = 1; s->n_past += 1;
+            s->last_launches = nodes; s->last_n = 1; s->n_past += 1;
             return;
         }
     }
@@ -599,6 +602,11 @@ static b200_session *start_session_tp(b200_session *s) {
                  m->gqa_loc % 32 == 0 && m->e_loc % 32 == 0 && hp.context_size % 8 == 0;
     B200_CHECK(cudaDeviceSynchronize());
     if (!s->mega_ok) { fprintf(stderr, "llm_b200: tensor-parallel session: geometry not supported by the fused decode schedule\n"); b200_session_free(s); return nullptr; }
+    // the ranks exchange attention rows in the cluster attention's epilogue, so every context bucket must fit it; the largest one is n_ctx itself
+    if (!attn_fused_fits((int)n_ctx, m->hd)) {
+        fprintf(stderr, "llm_b200: tensor-parallel session: context_size %d not supported by the fused decode attention (shared memory)\n", (int)n_ctx);
+        b200_session_free(s); return nullptr;
+    }
     return s;
 }
 
@@ -834,7 +842,7 @@ int b200_session_tp_set_nowait(b200_session *s, int32_t nowait) {     // measure
     B200_CHECK(cudaStreamSynchronize(rt().stream));
     s->dp.tp.nowait = nowait < 0 ? 0 : nowait > 2 ? 2 : nowait;
     decode_set_tp(s->dp.tp, rt().stream);
-    for (auto &g : s->graphs) cudaGraphExecDestroy(g.second);
+    for (auto &g : s->graphs) cudaGraphExecDestroy(g.exec);
     s->graphs.clear();
     return B200_OK;
 }
@@ -850,7 +858,7 @@ void b200_session_free(b200_session *s) {
     if (!s) return;
     B200_CHECK(cudaStreamSynchronize(rt().stream));
     if (s->h_n_past) B200_CHECK(cudaFreeHost(s->h_n_past));
-    for (auto &g : s->graphs) cudaGraphExecDestroy(g.second);
+    for (auto &g : s->graphs) cudaGraphExecDestroy(g.exec);
     if (s->tp_slab) {                                    // tensor-parallel session: the exchange slab and the peers' mappings
         for (int p = 0; p < TP_MAX; p++) if (s->tp_peer_map[p]) cudaIpcCloseMemHandle(s->tp_peer_map[p]);
         B200_CHECK(cudaFree(s->tp_slab)); B200_CHECK(cudaFree(s->tp_state));

@@ -24,6 +24,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from conftest import fingerprint  # noqa: E402
 import test_gpu_kquants as TK  # noqa: E402
+import test_gpu_long_context as TLC  # noqa: E402
 import test_gpu_neox as TN  # noqa: E402
 import test_kquants_lane_arithmetic as TL  # noqa: E402
 import test_oracle_kquants as TOK  # noqa: E402
@@ -106,6 +107,12 @@ def main():
             schedule(f"gpt2/{name}/lm_head={lm_head}", ref.gpt2(hp, tens, n_threads=8, n_batch=64), synth.make_tokens(hp, 60), TN.SCHEDULES["gpt2"])
     hp, tens = synth.make_gpt2(TN.GPT2_117M_3L, B.Q4_0, orc.quantize)
     schedule("gpt2_117m", ref.gpt2(hp, tens, n_threads=8, n_batch=64), synth.make_tokens(hp, 40), TN.SCHEDULES["gpt2_117m"])
+
+    # ---- tests/test_gpu_long_context.py
+    hp, tens = synth.make_neox(TLC.NEOX_LONG_CFG, B.Q4_0, orc.quantize)
+    schedule("neox_long/par/q4_0", ref.neox(hp, tens, n_threads=8, n_batch=512), synth.make_tokens(hp, 4096), TLC.LONG_CTX_SCHEDULE)
+    hp, tens = synth.make_gpt2(TLC.GPT2_LONG_CFG, B.Q8_0, orc.quantize)
+    schedule("gpt2_long/q8_0", ref.gpt2(hp, tens, n_threads=8, n_batch=512), synth.make_tokens(hp, 4096), TLC.LONG_CTX_SCHEDULE)
 
     with open(os.path.join(GOLDEN, "reference_outputs.json"), "w") as f:
         f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(v)}" for k, v in sorted(rec.items())) + "\n}\n")
